@@ -11,6 +11,7 @@ Every step draws FRESH weight samples (the reference draws new eps on every forw
     python bench.py --impl reference --steps K --warmup W    # the UNMODIFIED reference (baseline/_ref) on host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # N > 1: one rank per GPU, samples sharded
     python bench.py --config c4 ...                          # BASELINE.json configs[3]: ResNet-50 Flipout 3x224x224, N=32
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's mean / var as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  metric = MC image-samples/sec = B*N / t_step.
 The HEADLINE line is the fp32 model (fp32 parameters and activations -> tcgen05 kind::tf32 operands, the reference's
@@ -27,6 +28,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree: it writes nothing there
 
 CONFIGS = {
     # name: (arch, layer type, image, batch, MC samples, classes, metric, workload text)
@@ -223,17 +225,18 @@ def measure(args, cfg, dtype, dev, world, rank, local, want_roofline):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms per step, what the last step returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms) / steps
+        return float(ms) / steps, last
 
     if args.profile:          # under ncu: W warm-up passes + K steps of the device-resident step, nothing else
         for _ in range(args.warmup + args.steps):
@@ -245,17 +248,18 @@ def measure(args, cfg, dtype, dev, world, rank, local, want_roofline):
     sampler = ClockSampler(local)
     sampler.start()
     l0 = _native.launch_count
-    ms_step = timed(step_device, args.steps)
+    ms_step, (mean, var) = timed(step_device, args.steps)
     launches = _native.launch_count - l0
+    outputs = {"mean": mean.cpu(), "var": var.cpu()}          # [B, C] fp32 each, what mc_predict hands its caller
     sampler.stop_flag = True
     sampler.join(timeout=2)
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     out = {"ms_per_step": ms_step, "value": B * N_MC / (ms_step * 1e-3), "e2e_ms": ms_e2e,
            "e2e": {"value": B * N_MC / (ms_e2e * 1e-3), "unit": "image-samples/s", "ms_per_step": ms_e2e,
                    "h2d_bytes_per_step": x_host.numel() * 4, "d2h_bytes_per_step": 2 * B * classes * 4},
-           "gpu_launches": launches, "clocks": sampler.summary(), "chunk": chunk}
+           "gpu_launches": launches, "clocks": sampler.summary(), "chunk": chunk, "outputs": outputs}
     if not want_roofline:
         return out
 
@@ -350,6 +354,17 @@ def measure(args, cfg, dtype, dev, world, rank, local, want_roofline):
     return out
 
 
+def dump_outputs(dirname, by_dtype):
+    """DIR/<dtype>_<output>.npy (float32) of the last timed step of every model dtype that was measured.  The inputs
+    (image batch, parameters, Philox seed and sample offsets) depend only on the arguments, so two builds run with the
+    same arguments can be compared array for array."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for dt, outs in by_dtype.items():
+        for name, t in outs.items():
+            np.save(os.path.join(dirname, f"{dt}_{name}.npy"), t.float().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -385,6 +400,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {("fp32" if dt == torch.float32 else "bf16"): r["outputs"] for dt, r in res_by.items()})
     head = res_by[dtypes[0]]
     name = {torch.float32: "tf32 (fp32 parameters and activations, tcgen05 kind::tf32)", torch.bfloat16: "bf16"}
     line = {
@@ -430,7 +447,14 @@ if __name__ == "__main__":
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from python instead of replaying a CUDA graph")
     ap.add_argument("--no-fuse", action="store_true", help="keep BatchNorm/ReLU/residual as separate PyTorch kernels")
     ap.add_argument("--profile", action="store_true", help="profiling mode (ncu): only warmup+steps device steps, no JSON")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the predictive mean and variance of the last timed step as "
+                         "DIR/<dtype>_{mean,var}.npy (float32, [B, C])")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.profile):
+        ap.error("--dump-outputs writes the outputs of the timed B200 steps: not with --impl reference or --profile")
     if a.impl == "reference":
         run_reference(a)
     else:

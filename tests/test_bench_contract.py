@@ -1,10 +1,12 @@
 """CPU: the reference arm of bench.py (`--impl reference`: the reference's arithmetic on the host cores) prints ONE JSON
-line with the contract's keys; and `bench.py` without a GPU refuses to run the B200 arm instead of falling back."""
+line with the contract's keys; and `bench.py` without a GPU refuses to run the B200 arm instead of falling back.
+GPU: `--dump-outputs` writes the same arrays for the same arguments."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -37,3 +39,32 @@ def test_b200_arm_refuses_to_run_without_a_gpu():
                        capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"],
+                                  ["--profile", "--dump-outputs", "out"]])
+def test_bench_rejects_bad_arguments(args, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                       timeout=600, cwd=tmp_path)
+    assert r.returncode == 2 and "error:" in r.stderr
+    assert not list(tmp_path.iterdir())
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_for_the_same_arguments(tmp_path):
+    """--dump-outputs writes the last timed step's mean / var; two runs with the same arguments agree bit for bit"""
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--dtype", "fp32",
+                            "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900,
+                           cwd=tmp_path)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])["steps"] == 2
+        dumps.append({f.name: np.load(f) for f in sorted(d.iterdir())})
+    a, b = dumps
+    assert sorted(a) == ["fp32_mean.npy", "fp32_var.npy"]
+    for name in a:
+        assert a[name].dtype == np.float32 and a[name].shape == (128, 10), name
+        assert np.array_equal(a[name], b[name]), name
+    assert np.allclose(a["fp32_mean.npy"].sum(-1), 1.0, atol=1e-5) and (a["fp32_var.npy"] >= 0).all()

@@ -1,49 +1,46 @@
-"""CPU: the module-level port used for CPU timing (oracle/ref_model.py) replays the REFERENCE modules
-bit-exactly under the same seed.  Needs /root/reference (build container only; skipped on the GPU box)."""
+"""CPU: the module-level port used for CPU timing (oracle/ref_model.py) replays the REFERENCE modules bit-exactly under
+the same seed: same parameters and input, torch.manual_seed(5), then the port's forward must equal the reference
+module's output stored in tests/golden/port.npz (minted by tests/golden/make_golden_port.py)."""
 import os
-import subprocess
-import sys
 
+import numpy as np
 import pytest
+import torch
+import torch.nn as nn
 
-REF = "/root/reference"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-SCRIPT = r'''
-import sys
-sys.path.insert(0, "/root/reference"); sys.dont_write_bytecode = True
-sys.path.insert(1, %r)
-import torch, torch.nn as nn
-import bayesian_torch.layers as RL
-assert RL.__file__.startswith("/root/reference")
 from oracle.ref_model import OracleBayesLayer
-torch.set_num_threads(1)
-for flip in (False, True):
-    for det, x in ((nn.Conv2d(8, 12, 3, stride=2, padding=1), torch.randn(3, 8, 9, 9)),
-                   (nn.Linear(20, 7), torch.randn(5, 20)),
-                   (nn.Conv1d(4, 6, 3, padding=1, bias=False), torch.randn(2, 4, 11))):
-        name = type(det).__name__ + ("Flipout" if flip else "Reparameterization")
-        kw = dict(bias=det.bias is not None)
-        if isinstance(det, nn.Linear):
-            ref = getattr(RL, name)(det.in_features, det.out_features, **kw)
-        else:
-            ks = det.kernel_size if len(det.kernel_size) > 1 else det.kernel_size[0]
-            ref = getattr(RL, name)(det.in_channels, det.out_channels, ks, stride=det.stride, padding=det.padding, **kw)
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+_Z = np.load(os.path.join(ROOT, "tests", "golden", "port.npz"))
+
+# (layer, deterministic module it replaces, input shape); the same list as tests/golden/make_golden_port.py
+CASES = [("Conv2d", lambda: nn.Conv2d(8, 12, 3, stride=2, padding=1), (3, 8, 9, 9)),
+         ("Linear", lambda: nn.Linear(20, 7), (5, 20)),
+         ("Conv1d", lambda: nn.Conv1d(4, 6, 3, padding=1, bias=False), (2, 4, 11))]
+
+
+@pytest.fixture
+def one_thread():
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    yield
+    torch.set_num_threads(n)
+
+
+def test_port_replays_reference_modules_bitexact(one_thread):
+    for flip, (kind, make, xshape) in ((f, c) for f in (False, True) for c in CASES):
+        name = kind + ("Flipout" if flip else "Reparameterization")
+        g = {k[len(f"port/{name}/"):]: torch.from_numpy(_Z[k]) for k in _Z.files if k.startswith(f"port/{name}/")}
+        assert g, f"{name} missing from tests/golden/port.npz"
+        x = g["x"]
+        assert tuple(x.shape) == xshape, name
+        det = make()
         port = OracleBayesLayer(det, flip)
-        w = "weight" if isinstance(det, nn.Linear) else "kernel"
-        port.mu_w.data.copy_(getattr(ref, "mu_" + w).data); port.rho_w.data.copy_(getattr(ref, "rho_" + w).data)
+        port.mu_w.data.copy_(g["mu_w"]); port.rho_w.data.copy_(g["rho_w"])
         if det.bias is not None:
-            port.mu_b.data.copy_(ref.mu_bias.data); port.rho_b.data.copy_(ref.rho_bias.data)
-        torch.manual_seed(5); y_ref, kl_ref = ref(x)
-        torch.manual_seed(5); y = port(x)
-        assert torch.equal(y, y_ref), name
-        assert abs(float(port.kl_loss()) - float(kl_ref)) < 1e-5 * abs(float(kl_ref)), name
-print("PORT-OK")
-'''
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
-def test_port_replays_reference_modules_bitexact():
-    r = subprocess.run([sys.executable, "-c", SCRIPT % ROOT], capture_output=True, text=True, cwd="/tmp",
-                       env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
-    assert r.returncode == 0 and "PORT-OK" in r.stdout, r.stdout + r.stderr
+            port.mu_b.data.copy_(g["mu_b"]); port.rho_b.data.copy_(g["rho_b"])
+        torch.manual_seed(5)
+        y = port(x)
+        assert torch.equal(y, g["y"]), f"{name}: max abs {float((y - g['y']).abs().max())}"
+        kl_ref = float(g["kl"])
+        assert abs(float(port.kl_loss()) - kl_ref) < 1e-5 * abs(kl_ref), name
