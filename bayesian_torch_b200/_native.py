@@ -76,6 +76,9 @@ SYMBOLS = [
     ("bt_mc_accumulate_ex", _i, [_vp, _i, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp, _i, _vp]),
     ("bt_mc_uncertainty", _i, [_vp, _vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp, _vp]),
     ("bt_mc_finalize", _i, [_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp, _vp]),
+    ("bt_mc_accumulate_large", _i, [_vp, _i, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _vp, _vp, _i, _vp, _vp]),
+    ("bt_mc_regression_accumulate", _i, [_vp, _i, ctypes.c_int32, _i64, _vp, _i, _vp]),
+    ("bt_mc_regression_finalize", _i, [_vp, _i64, ctypes.c_int32, _vp, _vp, _vp]),
     ("bt_im2col2d", _i, [_vp, _i, _i64] + [ctypes.c_int32] * 3 + [ctypes.POINTER(ctypes.c_int64)] + [ctypes.c_int32] * 9 + [_vp, _vp]),
     ("bt_lstm_cell", _i, [_vp] * 7 + [_i] + [ctypes.c_int32] * 4 + [_vp]),
     ("bt_maxpool2d_nhwc", _i, [_vp, _i, _i64] + [ctypes.c_int32] * 9 + [_vp, _vp]),
@@ -269,17 +272,58 @@ def rng_export(what, out, rows, cols, taps, cols_per_group, seed, layer_key, sam
     return out
 
 
+MC_WARP_MAX_CLASSES = 1024     # bt_mc_accumulate_ex holds a row in one warp's registers; wider rows take the large-C path
+
+
 def mc_accumulate(logits, n_samples, batch, sums, accumulate, entropy_sum=None):
+    """logits: contiguous [S * batch, C] (batch = rows per sample); sums fp32 [2, batch, C], entropy_sum fp32 [batch]"""
     lib = load()
     require_cuda(logits, "logits")
     dev = logits.device
+    n_classes = int(logits.shape[-1])
     global launch_count
+    if n_classes > MC_WARP_MAX_CLASSES:
+        ws = torch.empty(2 * int(n_samples) * int(batch), dtype=torch.float32, device=dev)
+        launch_count += 2
+        with torch.cuda.device(dev):
+            _check(lib.bt_mc_accumulate_large(_ptr(logits), dtype_code(logits, "logits"), int(n_samples), int(batch),
+                                              n_classes, _ptr(sums), _ptr(entropy_sum), int(bool(accumulate)), _ptr(ws),
+                                              _stream(dev)))
+        return sums
     launch_count += 1
     with torch.cuda.device(dev):
         _check(lib.bt_mc_accumulate_ex(_ptr(logits), dtype_code(logits, "logits"), int(n_samples), int(batch),
-                                       int(logits.shape[-1]), _ptr(sums), _ptr(entropy_sum), int(bool(accumulate)),
+                                       n_classes, _ptr(sums), _ptr(entropy_sum), int(bool(accumulate)),
                                        _stream(dev)))
     return sums
+
+
+def mc_regression_accumulate(y, n_samples, sums, accumulate):
+    """y: the S samples' outputs, each sample's block of n elements contiguous in memory (sample-major);
+    sums: fp64 [2 * n]"""
+    lib = load()
+    require_cuda(y, "y")
+    if sums.dtype != torch.float64 or sums.numel() * int(n_samples) != 2 * y.numel():
+        raise ValueError("mc_regression_accumulate: sums must be float64 [2 * elements per sample]")
+    dev = y.device
+    global launch_count
+    launch_count += 1
+    with torch.cuda.device(dev):
+        _check(lib.bt_mc_regression_accumulate(_ptr(y), dtype_code(y, "y"), int(n_samples), sums.numel() // 2,
+                                               _ptr(sums), int(bool(accumulate)), _stream(dev)))
+    return sums
+
+
+def mc_regression_finalize(sums, n_total, mean, var):
+    """fp64 sums [2 * n] -> fp32 mean [n], var [n] (or None), in the sums' element order"""
+    lib = load()
+    dev = sums.device
+    global launch_count
+    launch_count += 1
+    with torch.cuda.device(dev):
+        _check(lib.bt_mc_regression_finalize(_ptr(sums), sums.numel() // 2, int(n_total), _ptr(mean), _ptr(var),
+                                             _stream(dev)))
+    return mean, var
 
 
 def mc_uncertainty(sums, entropy_sum, n_total, pred_entropy, mutual_info):

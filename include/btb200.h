@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define BT_VERSION 200 /* 0.2.0 */
+#define BT_VERSION 210 /* 0.2.1 */
 
 /* status codes */
 #define BT_OK 0
@@ -275,6 +275,31 @@ int bt_mc_uncertainty(const float* sums, const float* entropy_sum, int32_t batch
 /* sums [2,B,C] + total sample count -> mean [B,C], var [B,C] (predictive mean / variance). */
 int bt_mc_finalize(const float* sums, int32_t batch, int32_t n_classes, int32_t n_total,
                    float* mean, float* var, void* stream);
+
+/*
+ * bt_mc_accumulate_large -- bt_mc_accumulate_ex for any number of classes (bt_mc_accumulate_ex takes C <= 1024):
+ * logits [S * rows, C] (sample-major, each row of C classes contiguous) -> the same sums [2, rows, C] and optional
+ * entropy_sum [rows].  A dense head [S*B, C, *spatial] stored class-innermost is this with rows = B * prod(spatial).
+ * Two launches, each reading every logit once: the per-(sample, row) log-sum-exp and entropy, then the class sums.
+ * With `accumulate` the stored sums are the starting value and this call's samples are added to them in order.
+ * workspace: fp32, >= 2 * S * rows elements (S * rows without entropy_sum).  Deterministic (no atomics).
+ */
+int bt_mc_accumulate_large(const void* logits, int dtype, int32_t n_samples, int32_t rows, int32_t n_classes,
+                           float* sums, float* entropy_sum, int accumulate, float* workspace, void* stream);
+
+/*
+ * bt_mc_regression_accumulate -- Monte-Carlo moments of a regression output, elementwise:
+ *   sums[0, i] (+)= sum_s y[s * n + i],   sums[1, i] (+)= sum_s y[s * n + i]^2      (i < n_elem)
+ * y: the S samples' outputs, sample s occupying elements [s*n, (s+1)*n) in memory order (fp32 or bf16); sums fp64 [2, n].
+ * fp64 keeps the variance of outputs with a large mean and a small spread (fp32 sum y^2 / N - mean^2 cancels).
+ * Samples are added in order; the result has y's memory order, so a caller gets the output's strides for free.
+ */
+int bt_mc_regression_accumulate(const void* y, int dtype, int32_t n_samples, int64_t n_elem, double* sums,
+                                int accumulate, void* stream);
+
+/* fp64 sums [2, n] + total sample count -> fp32 mean [n], var [n] (var >= 0; var may be NULL). */
+int bt_mc_regression_finalize(const double* sums, int64_t n_elem, int32_t n_total, float* mean, float* var,
+                              void* stream);
 
 /*
  * bt_maxpool2d_nhwc -- channels-last 2-D max pooling (floor mode, dilation 1) of x [n_img, H, W, C] into

@@ -119,6 +119,20 @@ def main():
         _native.maxpool2d_nhwc(xp, (3, 3), (2, 2), (1, 1))
         torch.cuda.synchronize()
         print("aux kernels ok", flush=True)
+    if want("mc"):
+        # large-C softmax moments (two kernels, chunk accumulate) and the fp64 regression moments + finalize
+        logits = torch.randn(3 * 4, 1500, device=DEV).to(bf)
+        sums, ent = torch.empty(2, 4, 1500, device=DEV), torch.empty(4, device=DEV)
+        _native.mc_accumulate(logits[:8], 2, 4, sums, accumulate=False, entropy_sum=ent)
+        _native.mc_accumulate(logits[8:], 1, 4, sums, accumulate=True, entropy_sum=ent)
+        y = torch.randn(3 * 1000, device=DEV)
+        rs = torch.empty(2 * 1000, dtype=torch.float64, device=DEV)
+        _native.mc_regression_accumulate(y, 3, rs, accumulate=False)
+        _native.mc_regression_accumulate(y[1:2998], 3, torch.empty(2 * 999, dtype=torch.float64, device=DEV), False)
+        mean, var = torch.empty(1000, device=DEV), torch.empty(1000, device=DEV)
+        _native.mc_regression_finalize(rs, 3, mean, var)
+        torch.cuda.synchronize()
+        print("mc head kernels ok", flush=True)
 
 
 if __name__ == "__main__":
